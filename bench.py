@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this engine (one rank per GPU)
     python bench.py --impl reference --gpus N ...            # the reference's CPU path, host cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's results (dump_outputs)
 
 Workload (config.workload): the synthetic cube scene of BASELINE.json configs[3],
 500 cameras / 200k points / 2M observations (exactly 10 observations per point), which fits
@@ -467,6 +468,56 @@ def run_extras(pk, clocks_mhz, with_cpu):
 
 
 # --------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path returned, for comparing two builds output for output
+# --------------------------------------------------------------------------------------
+DUMP_BUDGET_BYTES = 64 << 20
+# row caps of the two outputs that outgrow the budget at C4 (2M reprojection errors, ~4M matches); the rest is whole
+DUMP_MAX_ROWS = {"ba_reprojection_errors": 1 << 20, "matches": 1 << 19}
+
+
+def sample_rows(n, max_rows, seed=0):
+    """Sorted indices of a fixed sample of `max_rows` out of `n` rows (all of them when n <= max_rows): the same
+    indices for the same n, whatever the values, so two builds that agree on the shapes are compared row for row."""
+    if n <= max_rows:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, max_rows, replace=False))
+
+
+def dump_outputs(dirname, ba, match_lists, pairs):
+    """Write one step's results as DIR/<name>.npy, float64:
+
+    ba_summary              [initial cost, final cost, LM iterations]
+    ba_points, ba_rig_instances, ba_rig_cameras, ba_cam_params   the solved parameters, whole
+    ba_reprojection_errors  rows sample_rows(N_obs, ...) of the (N_obs, 3) reprojection errors
+    match_counts            matches of every pair, in the order of the pair list
+    matches                 rows sample_rows(total, ...) of (image 1, image 2, feature 1, feature 2), the match lists of
+                            the pair list concatenated in its order
+    """
+    s = ba["summary"]
+    rep = ba["reprojection_errors"]
+    counts = np.array([len(match_lists[p]) for p in pairs], dtype=np.int64)
+    rows = np.concatenate([match_lists[p] for p in pairs]) if pairs else np.zeros((0, 2), dtype=np.int64)
+    keep = sample_rows(len(rows), DUMP_MAX_ROWS["matches"])
+    pair_of = np.searchsorted(np.cumsum(counts), keep, side="right")
+    arrays = {
+        "ba_summary": [s["initial_cost"], s["final_cost"], s["iterations"]],
+        "ba_points": ba["points"], "ba_rig_instances": ba["inst"], "ba_rig_cameras": ba["rigcam"],
+        "ba_cam_params": ba["cam_params"],
+        "ba_reprojection_errors": rep[sample_rows(len(rep), DUMP_MAX_ROWS["ba_reprojection_errors"])],
+        "match_counts": counts,
+        "matches": np.column_stack([np.asarray(pairs, dtype=np.int64).reshape(-1, 2)[pair_of], rows[keep]]),
+    }
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BUDGET_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_BUDGET_BYTES))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+    return sorted(arrays)
+
+
+# --------------------------------------------------------------------------------------
 # GPU arm
 # --------------------------------------------------------------------------------------
 def main():
@@ -478,8 +529,14 @@ def main():
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the BA solution and match lists of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the CUDA arm (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -580,12 +637,16 @@ def main():
         tot, ker = match_resident()
         mt_dev_ms += tot
         mt_kernel_ms += ker
-        dte, _ = match_e2e()
+        dte, matches = match_e2e()
         mt_wall += dte
     barrier()
     t_total = time.perf_counter() - t_begin
     clk = clocks.stop()
     launches = L.osfm_kernel_launch_count() - launches0
+    if args.dump_outputs:
+        matches = odist.gather_pair_results(matches, world)   # the pair list is sharded over the ranks
+        if rank == 0:
+            dump_outputs(args.dump_outputs, res, matches, pairs)
 
     # max over ranks
     vals = torch.tensor([t_total, ba_dev_ms, ba_wall, mt_dev_ms, mt_kernel_ms, mt_wall, ba_run_s], dtype=torch.float64, device="cuda")

@@ -1,18 +1,18 @@
-"""Fixture of the reference's known-answer test for the WORDS matcher (opensfm/test/test_matching.py:23-70), made HERE
-from the reference's own vocabulary file (it cannot travel to the GPU box):
+"""Fixture of the reference's known-answer test for the WORDS matcher (opensfm/test/test_matching.py:23-70), made from
+the reference's own vocabulary file, which is not part of this repository:
 
-    python tests/golden/make_words_golden.py        # reads /root/reference/opensfm/data/bow/bow_hahog_root_uchar_10000.npz
+    python tests/golden/make_words_golden.py <OpenSfM checkout>/opensfm/data/bow/bow_hahog_root_uchar_10000.npz
 
 Features as in `example_features` (seeded), their `bow_words_to_match` = 50 closest visual words computed the way
 opensfm/bow.py `map_to_words(..., "BRUTEFORCE")` does (cv2 BruteForce knnMatch against the vocabulary; the test itself
 asks for FLANN, the approximate version of the same query).  Saved: the seed and the word matrices."""
 import os
+import sys
 
 import cv2
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-BOW = "/root/reference/opensfm/data/bow/bow_hahog_root_uchar_10000.npz"
 SEED, NFEATURES, NUM_WORDS = 0, 1000, 50
 
 
@@ -26,7 +26,7 @@ def example_features(seed=SEED, nfeatures=NFEATURES):
 
 
 if __name__ == "__main__":
-    words = np.load(BOW)["words"].astype(np.float32)
+    words = np.load(sys.argv[1])["words"].astype(np.float32)
     f1, f2 = example_features()
     matcher = cv2.DescriptorMatcher_create("BruteForce")
 

@@ -265,7 +265,7 @@ def test_degenerate_inputs():
         bundle.solve(pb3)
 
 
-def test_kernel_variants_agree():
+def test_kernel_variants_agree(tmp_path):
     """The default path (persistent fp64 tensor-core segment Schur, pipelined PCG with S resident in shared memory) and the
     kernels it replaces (per-point ba_schur, SIMT segment kernel, classic / streamed PCG) must give the same solve."""
     import os
@@ -284,7 +284,7 @@ def test_kernel_variants_agree():
     variants = {"default": {}, "generic_schur": {"OSFM_BA_SEGMENT_SCHUR": "0"}, "simt_seg_schur": {"OSFM_BA_SCHUR_MMA": "0"}, "cta_per_segment_schur": {"OSFM_BA_SCHUR_PIPE": "0"}, "generic_linearize": {"OSFM_BA_LIN_SPECIAL": "0"}, "undeflated_pcg": {"OSFM_BA_PCG_DEFLATE": "0"}, "explicit_model_change": {"OSFM_BA_MODEL_CHANGE_EXPLICIT": "1"}, "classic_pcg": {"OSFM_BA_PCG_PIPELINED": "0"}, "b128_barrier": {"OSFM_BA_PCG_B128": "1"},
                 "streamed_pcg": {"OSFM_BA_PCG_PIPELINED": "0", "OSFM_BA_PCG_RESIDENT": "0"}}
     for name, extra in variants.items():
-        path = "/tmp/osfm_variant_%s.npy" % name
+        path = str(tmp_path / ("%s.npy" % name))
         env = dict(os.environ, **extra)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env, timeout=600)
         out[name] = np.load(path)

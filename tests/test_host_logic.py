@@ -227,3 +227,72 @@ def test_bench_submodel_workload_host_logic(monkeypatch):
     assert cams == [14, 14, 15, 13] and seen["solve"] == 8            # warm-up + timed solve per submodel
     assert seen["problems"] == [(50, 4, 50 + sum(cams))] * 2          # 50 GPS terms + one relative motion per (submodel, shot)
     assert out["alignment_terms"] == 50 + sum(cams)
+
+
+def _bench():
+    import importlib
+
+    if ROOT not in sys.path:
+        sys.path.insert(0, ROOT)
+    return importlib.import_module("bench")
+
+
+def test_bench_dump_outputs_layout_and_sample(tmp_path):
+    """bench.dump_outputs: float64 .npy files, matches tagged with their pair in pair-list order, and a sample of the
+    outgrown outputs that depends on the row count only."""
+    bench = _bench()
+    rng = np.random.default_rng(1)
+    pairs = [(0, 1), (0, 2), (1, 2)]
+    lists = {(0, 1): np.array([[0, 3], [2, 1]], np.int32), (0, 2): np.zeros((0, 2), np.int32),
+             (1, 2): np.array([[5, 4]], np.int32)}
+    ba = {"summary": {"initial_cost": 2.0, "final_cost": 1.0, "iterations": 7}, "points": rng.normal(size=(4, 3)),
+          "inst": rng.normal(size=(3, 6)), "rigcam": np.zeros((1, 6)), "cam_params": rng.normal(size=9),
+          "reprojection_errors": rng.normal(size=(10, 3))}
+    names = bench.dump_outputs(str(tmp_path / "out"), ba, lists, pairs)
+    got = {n: np.load(str(tmp_path / "out" / (n + ".npy"))) for n in names}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got["ba_summary"].tolist() == [2.0, 1.0, 7.0]
+    assert np.array_equal(got["ba_points"], ba["points"]) and np.array_equal(got["ba_cam_params"], ba["cam_params"])
+    assert np.array_equal(got["ba_reprojection_errors"], ba["reprojection_errors"])
+    assert got["match_counts"].tolist() == [2, 0, 1]
+    assert got["matches"].tolist() == [[0, 1, 0, 3], [0, 1, 2, 1], [1, 2, 5, 4]]
+
+    keep = bench.sample_rows(1000, 100)
+    assert len(keep) == 100 and np.all(np.diff(keep) > 0) and keep[-1] < 1000
+    assert np.array_equal(keep, bench.sample_rows(1000, 100))
+    assert np.array_equal(bench.sample_rows(50, 100), np.arange(50))
+
+
+def test_bench_rejects_zero_steps():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True,
+                         text=True, timeout=120, cwd=ROOT)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_the_timed_results(tmp_path):
+    """`bench.py --dump-outputs` writes what the timed steps computed: the BA solution and the match lists the public
+    API returns for the same workload."""
+    import json
+
+    from opensfm_b200 import matching
+
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny", "--steps", "2",
+                          "--warmup", "1", "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-3000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 2
+    bench = _bench()
+    pb, feats, pairs, _ = bench.build_workload("tiny")
+    got = {f[:-4]: np.load(str(tmp_path / f)) for f in os.listdir(str(tmp_path))}
+    ref = bundle.solve(pb)
+    assert got["ba_summary"][2] == ref["summary"]["iterations"]
+    assert abs(got["ba_summary"][1] - ref["summary"]["final_cost"]) <= 1e-12 * ref["summary"]["final_cost"]
+    assert np.abs(got["ba_points"] - ref["points"]).max() < 1e-9
+    assert np.abs(got["ba_reprojection_errors"] - ref["reprojection_errors"]).max() < 1e-9
+    pm = matching.PairMatcher()
+    pm.add_many([(i, f.astype(np.uint8)) for i, f in enumerate(feats)], uint8_is_l2=True)
+    lists = pm.match_pairs(pairs, {"lowes_ratio": 0.8})
+    assert got["match_counts"].tolist() == [len(lists[p]) for p in pairs]
+    want = np.concatenate([np.column_stack([np.tile(p, (len(lists[p]), 1)), lists[p]]) for p in pairs])
+    assert np.array_equal(got["matches"], want)
